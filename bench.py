@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the grayskull hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4|c5|ops|match|tmatch] [--impl reference]
+                    [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1] ("c2"): gs_blur r=5 + gs_sobel on 4096x4096 synthetic
 uint8 frames, batch 256 per GPU (weak scaling: every rank processes its own 256 frames; frames are
@@ -21,6 +22,17 @@ One JSON line on stdout (rank 0):
   cpu_baseline  the reference's own C code (oracle/_ref, built from /root/reference) timed on this
              box's host cores on a bounded sample of the same workload
 With --impl reference the whole line is the reference CPU arm (rank 0 only).
+
+--steps K is the number of timed steps of the GPU arm.  The reference arm (--impl reference) runs at most K, as many
+as fit its time budget, and reports the count it ran.
+
+--dump-outputs DIR writes, right after the timed steps of the headline workload, what its last step computed
+(the arrays a caller of that path receives) as DIR/<name>.npy: float32 for 8/16-bit data, float64 for 32-bit
+words (exact), rows past a per-frame count zeroed.  DUMP_BYTES is shared out smallest output first, each taking all
+of itself or an equal part of what is left; an output larger than its part is replaced by a fixed sample, the
+sorted flat indices np.random.default_rng(0).integers(0, numel, k).  Inputs are seeded, so two builds run with the
+same arguments can be compared array for array.  c3, c4 and tmatch blur their seeded noise with the build's own
+gs_blur before timing, so a change to gs_blur also changes those workloads' inputs.  Rank 0 only.
 """
 import argparse
 import ctypes as C
@@ -45,6 +57,7 @@ W4, H4, B4 = 3840, 2160, 256                  # c4 (sf 1.1, scales 1..4, step 2,
 B5 = 1024                                     # c5: 8192 frames over 8 GPUs
 NWIN4 = 30016520                              # windows per UHD frame (SURVEY.md 8d; checked against the library)
 FALLBACK_HBM_GBS = 6650.0
+DUMP_BYTES = 60_000_000                       # --dump-outputs: array data of all files together (headers stay under 64 MB)
 NVLINK_GBS = 900.0                            # NVLink 5 per direction per GPU: the root's egress / ingress bound
 
 METRICS = {
@@ -428,7 +441,7 @@ def build_workload(cx, wl, batch):
                         "gs_sobel": (lambda: api.sobel_batch(blur, out=sob), px + 1.0 * n * (h - 2) * (w - 2))}
         if fused:
             W["variant_kernels"] = {"gs_blur_sobel_r5": (step_fused, px + 1.0 * n * (h - 2) * (w - 2))}
-        W.update(units=n * h * w, n=n, h=h, w=w, src=src, keep=(blur, sob))
+        W.update(units=n * h * w, n=n, h=h, w=w, src=src, keep=(blur, sob), outputs=lambda: {"blur": blur, "sobel": sob})
     elif wl == "c3":
         n, h, w = batch or B3, H3, W3
         noise = torch.randint(0, 256, (n, h, w), dtype=torch.uint8, device=dev)
@@ -444,7 +457,8 @@ def build_workload(cx, wl, batch):
                                                           NK3, T3, st()), "orb_extract_batch")
 
         W.update(step=step, kernels={"gs_orb_extract": (step, 2.0 * n * h * w + 48.0 * n * NK3)},
-                 units=n * h * w, n=n, h=h, w=w, src=src, keep=(sm, kps, cnt))
+                 units=n * h * w, n=n, h=h, w=w, src=src, keep=(sm, kps, cnt),
+                 outputs=lambda: {"scoremap": sm, "keypoints": _keypoints(kps, cnt), "keypoint_counts": cnt})
     elif wl == "c4":
         n, h, w = batch or B4, H4, W4
         cas = g.load_cascade()
@@ -468,7 +482,8 @@ def build_workload(cx, wl, batch):
 
         W.update(step=step, kernels={"gs_integral": (lambda: api.integral_batch(src, out=ii), 5.0 * n * h * w),
                                      "gs_lbp_detect": (lbp, 4.0 * n * h * w)},
-                 units=n * nwin, n=n, h=h, w=w, src=src, keep=(ii, rects, rc, cas), nwin=nwin)
+                 units=n * nwin, n=n, h=h, w=w, src=src, keep=(ii, rects, rc, cas), nwin=nwin,
+                 outputs=lambda: {"integral": ii, "rects": _valid_rows(rects, rc), "rect_counts": rc}, unsigned={"integral"})
     elif wl == "c5":
         # BASELINE configs[4]: blur -> sobel -> FAST/ORB -> integral + LBP on 1920x1080 frames, sharded by frame
         # (8192 frames over 8 GPUs = 1024 per GPU).  FAST and LBP both run on the sobel output (SURVEY.md 8d).
@@ -496,7 +511,10 @@ def build_workload(cx, wl, batch):
                     P["scale_factor"], P["min_scale"], P["max_scale"], P["step"], st())), 4.0 * px)}
         if hasattr(api, "blur_sobel_batch"):
             W["variant_kernels"] = {"gs_blur_sobel_r5": (lambda: api.blur_sobel_batch(src, R2, out=pipe.score), 2.0 * px)}
-        W.update(step=step, kernels=kern, units=n * h * w, n=n, h=h, w=w, src=src, keep=(pipe, up, cas))
+        W.update(step=step, kernels=kern, units=n * h * w, n=n, h=h, w=w, src=src, keep=(pipe, up, cas),
+                 outputs=lambda: {"sobel": pipe.sobel, "keypoints": _keypoints(pipe.kps, pipe.kcounts),
+                                  "keypoint_counts": pipe.kcounts, "rects": _valid_rows(pipe.rects, pipe.rcounts),
+                                  "rect_counts": pipe.rcounts})
     elif wl == "match":
         # SURVEY.md 8(f) N1: gs_match_orb over frame pairs (1250 x 1250 descriptors each, the c3 keypoint budget).
         # Not HBM-bound: 8 POPC per descriptor comparison on the 16-lane/clk/SM POPC path bounds it.
@@ -509,12 +527,14 @@ def build_workload(cx, wl, batch):
         k1[:, nd // 2:, 4:] = torch.randint(-2**31, 2**31 - 1, (npairs, nd - nd // 2, 8), dtype=torch.int32, device=dev, generator=gen)
         del flip
         cnt = torch.full((npairs,), nd, dtype=torch.int32, device=dev)
+        last = {}
 
         def step():
-            api.match_orb_batch(k1, cnt, k2, cnt, nd, 60.0)
+            last["matches"], last["counts"] = api.match_orb_batch(k1, cnt, k2, cnt, nd, 60.0)
 
         W.update(step=step, kernels={"gs_match_orb": (step, 2.0 * npairs * nd * 48 + 12.0 * npairs * nd)},
                  units=npairs * nd * nd, n=npairs, h=nd, w=nd, src=k1, keep=(k2, cnt),
+                 outputs=lambda: {"matches": _valid_rows(last["matches"], last["counts"]), "match_counts": last["counts"]},
                  metric=("256-bit descriptor comparisons/s, gs_match_orb 1250 x 1250 per frame pair", "Gcomparisons/s", 1e-9),
                  cfg={"workload": "match: gs_match_orb max_distance=60, 1250 x 1250 descriptors per pair, %d pairs per GPU" % npairs,
                       "pairs_per_gpu": npairs, "l2": "descriptor sets (%.0f MB per GPU) exceed the 126 MB L2" % (2 * npairs * nd * 48 / 1e6)})
@@ -528,13 +548,15 @@ def build_workload(cx, wl, batch):
         del noise
         tmpl = src[0, 500:500 + th, 900:900 + tw].contiguous()
         res = torch.empty((n, h - th + 1, w - tw + 1), dtype=torch.uint8, device=dev)
+        last = {}
 
         def step():
             api.match_template_batch(src, tmpl, out=res)
-            api.find_best_match_batch(res)
+            last["best"] = api.find_best_match_batch(res)
 
         W.update(step=step, kernels={"gs_match_template": (lambda: api.match_template_batch(src, tmpl, out=res), 2.0 * n * h * w)},
                  units=n * (h - th + 1) * (w - tw + 1) * tw * th, n=n, h=h, w=w, src=src, keep=(tmpl, res),
+                 outputs=lambda: {"match": res, "best_match": last["best"]},
                  metric=("squared differences/s, gs_match_template 32x32 template, 1920x1080 uint8", "Gtaps/s", 1e-9),
                  cfg={"workload": "tmatch: gs_match_template + gs_find_best_match, 32x32 template, 1920x1080, batch %d per GPU" % n,
                       "frames_per_gpu": n, "l2": "compute-bound; frames (%.0f MB per GPU) stream through L2" % (n * h * w / 1e6)})
@@ -584,6 +606,8 @@ def build_workload(cx, wl, batch):
 
         W.update(step=step, kernels=kernels, units=n * h * w * len(kernels), n=n, h=h, w=w, src=src,
                  keep=(out, half, odd, ii, hist, oth),
+                 outputs=lambda: {"out": out, "half": half, "resized_2560x1440": odd, "integral": ii, "histogram": hist,
+                                  "otsu": oth}, unsigned={"integral"},
                  metric=("Mpixels/s summed over the per-op table, 4096x4096 uint8", "Mpixels/s", 1e-6),
                  cfg={"workload": "ops: every stencil/resampling op once, 4096x4096 synthetic uint8, batch %d per GPU" % n,
                       "frames_per_gpu": n, "l2": "inputs (%.1f GiB per GPU) exceed the 126 MB L2" % (n * h * w / 2**30)})
@@ -595,14 +619,62 @@ def build_workload(cx, wl, batch):
     return W
 
 
-def measure(cx, wl, batch, steps, warmup, with_kernels=True):
-    """headline numbers of one workload: device-resident steps, per-entry-point table, roofline, clocks"""
+def _u32(t):
+    """int32-typed storage of unsigned 32-bit words -> their values as int64"""
+    import torch
+    return t.to(torch.int64) & 0xFFFFFFFF
+
+
+def _valid_rows(t, counts):
+    """(n, cap, k) records of which counts[i] are valid in frame i: the rows past the count zeroed (they hold
+    whatever an earlier step or allocation left there)"""
+    import torch
+    keep = torch.arange(t.shape[1], device=t.device)[None, :] < counts[:, None].to(torch.int64)
+    return t * keep[..., None].to(t.dtype)
+
+
+def _keypoints(kps, counts):
+    """(n, nkps, 12) struct gs_keypoint words -> x, y, response, angle, descriptor[8] as values (float64)"""
+    import torch
+    k = _valid_rows(kps, counts)
+    v = _u32(k).to(torch.float64)
+    v[..., 3] = k[..., 3].contiguous().view(torch.float32).to(torch.float64)
+    return v
+
+
+def dump_outputs(outputs, out_dir, unsigned=()):
+    """write each output as out_dir/<name>.npy (see the module docstring for dtypes and sampling).
+    unsigned: names of int32-typed outputs that hold unsigned 32-bit words"""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    os.makedirs(out_dir, exist_ok=True)
+    left, names = DUMP_BYTES, sorted(outputs, key=lambda n: outputs[n].numel())
+    for i, name in enumerate(names):
+        t = outputs[name]
+        dt = torch.float32 if t.element_size() <= 2 or t.dtype == torch.float32 else torch.float64
+        size = 4 if dt == torch.float32 else 8
+        k = min(t.numel(), left // (len(names) - i) // size)
+        if t.numel() > k:                        # sample first: only the k picked values are widened
+            idx = np.sort(np.random.default_rng(0).integers(0, t.numel(), k))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        if name in unsigned:
+            t = _u32(t)
+        np.save(os.path.join(out_dir, name + ".npy"), t.to(dt).cpu().numpy())
+        left -= k * size
+
+
+def measure(cx, wl, batch, steps, warmup, with_kernels=True, dump=None):
+    """headline numbers of one workload: device-resident steps, per-entry-point table, roofline, clocks.
+    dump: directory for the outputs of the last timed step (written before anything else reuses the buffers)"""
     W = build_workload(cx, wl, batch)
     metric, unit, scale = W["metric"]
     clocks = []
     l0 = cx.lib.gs_b200_launch_count()
     ms = cx.time_steps(W["step"], steps, warmup, clocks=clocks)
     launched = cx.lib.gs_b200_launch_count() - l0
+    if dump and cx.rank == 0:
+        dump_outputs(W["outputs"](), dump, W.get("unsigned", ()))
     out = {"metric": metric, "value": W["units"] * cx.world * steps / (ms * 1e-3) * scale, "unit": unit,
            "steps": steps, "warmup": warmup, "ms_per_step": ms / steps, "config": W["cfg"],
            "clocks": clocks[0] if clocks else None,
@@ -779,7 +851,7 @@ def gpu_main(args):
     cx = Ctx()
     torch = cx.torch
     wl = args.workload
-    res, W = measure(cx, wl, args.batch, args.steps, args.warmup)
+    res, W = measure(cx, wl, args.batch, args.steps, args.warmup, dump=args.dump_outputs)
     metric, unit, scale = W["metric"]
     out = {"metric": res["metric"], "value": res["value"], "unit": unit, "n_gpus": cx.world, "steps": args.steps,
            "warmup": args.warmup, "ms_per_step": res["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -862,7 +934,7 @@ def reference_main(args):
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps (--impl reference: at most this many, see above)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--workload", default="c2", choices=["c2", "c3", "c4", "c5", "ops", "match", "tmatch"])
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
@@ -879,7 +951,10 @@ if __name__ == "__main__":
     ap.add_argument("--shard-steps", type=int, default=2)
     ap.add_argument("--shard-chunks", type=int, default=4)
     ap.add_argument("--cpu-cores", type=int, default=0, help="cap the cores of the cpu_baseline sample (default: all)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "b200" or a.steps < 1):
+        ap.error("--dump-outputs needs the GPU arm and --steps >= 1")
     if a.impl == "reference":
         reference_main(a)
     else:

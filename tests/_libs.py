@@ -1,6 +1,7 @@
 """ctypes loaders shared by the tests: the oracle restatement, the real reference build
 (oracle/_ref, when present) and synthetic-input generators.  TEST INFRASTRUCTURE only."""
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -176,6 +177,232 @@ def ref():
         lib.ref_sort_keypoints.restype = None
         _cache["r"] = lib
     return _cache["r"]
+
+
+def digest(x):
+    """16-byte digest of an output or an input tuple: arrays by dtype, shape and bytes, Python ints as int64, floats
+    as float64 (exact for the c_float results), tuples / lists element by element, RefDigest as itself"""
+    if isinstance(x, RefDigest):
+        return x
+    h = hashlib.blake2b(digest_size=16)
+
+    def feed(v):
+        if isinstance(v, (tuple, list)):
+            h.update(b"(%d" % len(v))
+            for e in v:
+                feed(e)
+        elif isinstance(v, np.ndarray):
+            h.update(v.dtype.str.encode() + repr(v.shape).encode()); h.update(np.ascontiguousarray(v).tobytes())
+        elif isinstance(v, (bool, int, np.integer)):
+            h.update(b"i"); h.update(np.int64(v).tobytes())
+        elif isinstance(v, (float, np.floating)):
+            h.update(b"f"); h.update(np.float64(v).tobytes())
+        elif isinstance(v, str):
+            h.update(b"s" + v.encode())
+        else:
+            raise TypeError(type(v))
+    feed(x)
+    return RefDigest(h.digest())
+
+
+class RefDigest(bytes):
+    """a reference output known by its digest only (replayed from tests/golden/ref_digests.npz)"""
+
+
+def same(want, got):
+    """exact equality of a reference output (array, scalar or RefDigest) and an oracle output"""
+    return digest(want) == digest(got)
+
+
+REF_DIGESTS = os.path.join(ROOT, "tests", "golden", "ref_digests.npz")
+
+
+class RefRecord:
+    """The compiled reference (oracle/_ref/libgs_ref.so) as the differential tests see it: `R.blur(a, 5)` is what
+    the reference's gs_blur returns for that input.  By default every call is replayed from
+    tests/golden/ref_digests.npz: the stored entry must have been made from the same operation and inputs, and
+    its output digest is returned (compare with `same`).  With GS_REF_RECORD=1 and oracle/_ref built, the
+    reference itself is called, the test compares against its real outputs, and the stream is (re)written.
+
+    Two costs of storing digests instead of arrays: a replayed mismatch says which call differs, not where in the
+    output (re-run with GS_REF_RECORD=1 to compare real arrays); and the input digests pin the inputs the tests draw
+    from numpy's Generator streams, so a numpy release that changes those streams fails every call with "is not the
+    recorded one" until the file is re-recorded with the reference build."""
+
+    def __init__(self, name):
+        self.name, self.pos, self.rows = name, 0, []
+        self.record = os.environ.get("GS_REF_RECORD") == "1"
+        if self.record:
+            assert have_ref(), "GS_REF_RECORD=1 needs oracle/_ref/libgs_ref.so (make -C oracle REF=<reference tree>)"
+        else:
+            z = np.load(REF_DIGESTS)
+            self.stored = z[name]             # (calls, 2, 16) uint8: input digest, output digest
+
+    def __getattr__(self, op):
+        if op not in _REF_OPS:
+            raise AttributeError(op)
+        return lambda *args: self._call(op, args)
+
+    def _call(self, op, args):
+        key = digest((op,) + tuple(args))
+        if self.record:
+            out = _REF_OPS[op](ref(), *args)
+            self.rows.append((key, digest(out)))
+            return out
+        assert self.pos < len(self.stored), "%s: more reference calls than recorded (%s)" % (self.name, op)
+        k, out = bytes(self.stored[self.pos, 0]), bytes(self.stored[self.pos, 1])
+        assert k == key, "%s: call %d (%s%r) is not the recorded one" % (self.name, self.pos, op, tuple(
+            a if np.isscalar(a) else getattr(a, "shape", "...") for a in args))
+        self.pos += 1
+        return RefDigest(out)
+
+    def finish(self):
+        if not self.record:
+            assert self.pos == len(self.stored), "%s: %d of %d recorded calls made" % (self.name, self.pos, len(self.stored))
+            return
+        rows = np.frombuffer(b"".join(k + o for k, o in self.rows), np.uint8).reshape(-1, 2, 16)
+        old = dict(np.load(REF_DIGESTS)) if os.path.exists(REF_DIGESTS) else {}
+        old[self.name] = rows
+        np.savez_compressed(REF_DIGESTS, **old)
+
+
+def _into(fn, shape_of=lambda a: a.shape, fill=0):
+    """a reference call fn(dst, src, *args) that writes a uint8 image of shape shape_of(src)"""
+    def run(R, a, *args):
+        d = np.full(shape_of(a), fill, np.uint8)
+        getattr(R, fn)(img(d), img(a), *args)
+        return d
+    return run
+
+
+def _ref_resize(R, a, dw, dh):
+    d = np.empty((dh, dw), np.uint8)
+    R.gs_resize(img(d), img(a))
+    return d
+
+
+def _ref_integral(R, a):
+    ii = np.empty(a.shape, np.uint32)
+    R.gs_integral(img(a), ptr(ii))
+    return ii
+
+
+def _ref_fast(R, a, sm0, cap, t):
+    sm, k = sm0.copy(), np.zeros(cap, KP_DTYPE)
+    n = R.gs_fast(img(a), img(sm), ptr(k), cap, t)
+    return sm, k[:n]
+
+
+def _ref_orb(R, a, nk, t):
+    k, sm = np.zeros(nk, KP_DTYPE), np.zeros_like(a)
+    return k[:R.gs_orb_extract(img(a), ptr(k), nk, t, ptr(sm))]
+
+
+def _ref_sort(R, k):
+    k = k.copy()
+    R.ref_sort_keypoints(ptr(k), len(k))
+    return k
+
+
+def _ref_libm(fn, *cols):
+    f = getattr(C.CDLL("libm.so.6"), fn)
+    f.restype, f.argtypes = C.c_float, [C.c_float] * len(cols)
+    return np.array([f(*(float(c[i]) for c in cols)) for i in range(len(cols[0]))], np.float32)
+
+
+def _ref_lbp_detect(R, ii, mr, sf, mn, mx, st):
+    rr = np.zeros(mr, RECT_DTYPE)
+    return rr[:R.gs_lbp_detect(R.ref_frontalface(), ptr(ii), ii.shape[1], ii.shape[0], ptr(rr), mr, sf, mn, mx, st)]
+
+
+def _ref_match_orb(R, k1, k2, mm, md):
+    m = np.zeros(max(mm, 1), MATCH_DTYPE)
+    return m[:R.gs_match_orb(ptr(k1), len(k1), ptr(k2), len(k2), ptr(m), mm, md)]
+
+
+def _ref_histogram(R, a):
+    h = np.zeros(256, np.uint32)
+    R.gs_histogram(img(a), ptr(h))
+    return h
+
+
+def _ref_threshold(R, a, t):
+    x = a.copy()
+    R.gs_threshold(img(x), t)
+    return x
+
+
+def _ref_filter(R, a, k, norm):
+    d = np.zeros_like(a)
+    R.gs_filter(img(d), img(a), img(k), norm)
+    return d
+
+
+def _ref_match_template(R, a, tmpl):
+    rw, rh = a.shape[1] - tmpl.shape[1] + 1, a.shape[0] - tmpl.shape[0] + 1
+    rr = np.zeros((rh, rw), np.uint8)
+    R.gs_match_template(img(a), img(tmpl), img(rr))
+    p = R.gs_find_best_match(img(rr))
+    return rr, p.y * rw + p.x
+
+
+def _ref_find_best_match(R, r):
+    p = R.gs_find_best_match(img(r))
+    return p.x, p.y
+
+
+def _ref_blobs(R, a, nb):
+    labels, blobs = np.full(a.shape, 0x5555, np.uint16), np.zeros(nb, BLOB_DTYPE)
+    m = R.gs_blobs(img(a), ptr(labels), ptr(blobs), nb)
+    return labels, blobs[:m]
+
+
+def blobs_result(labels, blobs):
+    """(labels, defined gs_blob fields as an (n, 8) int64 array): what the blob tests compare"""
+    return labels, np.array(blob_fields(blobs), np.int64).reshape(-1, 8)
+
+
+def _ref_blob_corners(R, a, nb, j):
+    labels, blobs = _ref_blobs(R, a, nb)
+    c = np.zeros((4, 2), np.uint32)
+    R.gs_blob_corners(img(a), ptr(labels), ptr(blobs[j:j + 1]), ptr(c))
+    return c
+
+
+def _ref_perspective(R, src, dw, dh, c):
+    d = np.empty((dh, dw), np.uint8)
+    R.gs_perspective_correct(img(d), img(src), ptr(c))
+    return d
+
+
+_REF_OPS = {
+    "blur": _into("gs_blur"),
+    "adaptive": _into("gs_adaptive_threshold"),
+    "erode": _into("gs_erode"),
+    "dilate": _into("gs_dilate"),
+    "sobel77": _into("gs_sobel", fill=77),
+    "downsample": _into("gs_downsample", lambda a: (a.shape[0] // 2, a.shape[1] // 2)),
+    "resize": _ref_resize,
+    "integral": _ref_integral,
+    "fast": _ref_fast,
+    "orb_extract": _ref_orb,
+    "sort_keypoints": _ref_sort,
+    "libm_sinf": lambda R, xs: _ref_libm("sinf", xs),
+    "libm_atan2f": lambda R, ys, xs: _ref_libm("atan2f", ys, xs),
+    "lbp_detect": _ref_lbp_detect,
+    "lbp_window": lambda R, ii, x, y, s: R.gs_lbp_window(R.ref_frontalface(), ptr(ii), ii.shape[1], ii.shape[0], x, y, s),
+    "match_orb": _ref_match_orb,
+    "histogram": _ref_histogram,
+    "otsu": lambda R, a: int(R.gs_otsu_threshold(img(a))),
+    "threshold": _ref_threshold,
+    "filter": _ref_filter,
+    "match_template": _ref_match_template,
+    "find_best_match": _ref_find_best_match,
+    "blobs": lambda R, a, nb: blobs_result(*_ref_blobs(R, a, nb)),
+    "blob_corners": _ref_blob_corners,
+    "perspective": _ref_perspective,
+    "orientation": lambda R, a, x, y, r: R.gs_compute_orientation(img(a), x, y, r),
+}
 
 
 class HostCascade:
